@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # reference CPU arithmetic (rank 0)
+    python bench.py --steps K --warmup W --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
 
 Workload (config.workload): synthetic 1.3M cells x 2000 HVGs CSR (~5 % dense), n_pcs=50, k=15 — the
 configuration BASELINE.json's metric is quoted on; it fits one B200.  One "step" = one full pass of the
@@ -52,7 +53,11 @@ def parse_args():
     p.add_argument("--knn-queries", type=int, default=8192)
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-parity", action="store_true", help="skip the host-side fp64 parity checks after the timed region")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (see dump_outputs)")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    return a
 
 
 def workload_config(a, n_gpus):
@@ -231,6 +236,47 @@ def parity_checks(a, out, x_host, labels, row_range, n_rows_sample: int = 2000):
     return res
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(a, out, directory):
+    """Writes what one step of the timed path returns to a caller, as DIR/<name>.npy in float32 or float64, so that two
+    builds run with the same arguments (hence the same synthetic input) can be compared output for output.  Per-cell
+    outputs are kept for a seeded sample of cells that depends on --n-cells alone (`rows`, sorted), sized so that the
+    files stay under 64 MiB; the connectivities are those rows of the CSR with their column indices sorted."""
+    import torch
+    from scipy import sparse
+
+    from scanpy_b200 import _ops
+
+    n, d, k, g = a.n_cells, a.n_pcs, a.k, a.n_genes
+    fixed = 4 * d * g + 8 * g + 16 * d + 8
+    per_row = 8 + 4 * d + 16 * k + 8 + 12 * 4 * k    # row id, X_pca, kNN indices + distances, label, ~4k connectivities
+    m = min(n, max(1, (DUMP_BYTES - fixed) // per_row))
+    rows = np.sort(np.random.RandomState(0).choice(n, m, replace=False))
+    sel = torch.from_numpy(rows).to("cuda")
+    x_pca, knn_idx, knn_dist, member = _ops._to_host(out["X_pca"].index_select(0, sel), out["knn_idx"].index_select(0, sel),
+                                                     out["knn_dist"].index_select(0, sel), out["membership"].index_select(0, sel))
+    indptr, indices, data = _ops._to_host(*out["conn"])
+    conn = sparse.csr_matrix((data, indices, indptr), shape=(n, n))[rows].sorted_indices()
+    pca = out["pca"]
+    arrays = dict(rows=rows.astype(np.float64), X_pca=x_pca, pca_components=_ops._to_host(pca["components"]),
+                  pca_variance=pca["variance"], pca_variance_ratio=pca["variance_ratio"], pca_mean=pca["mean"],
+                  knn_indices=knn_idx.astype(np.float64), knn_distances=knn_dist,
+                  connectivities_indptr=conn.indptr.astype(np.float64), connectivities_indices=conn.indices.astype(np.float64),
+                  connectivities_data=conn.data, leiden_membership=member.astype(np.float64),
+                  modularity=np.float64(out["modularity"]))
+    total = sum(np.asarray(v).nbytes for v in arrays.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, v in arrays.items():
+        v = np.asarray(v)
+        assert v.dtype in (np.float32, np.float64), (name, v.dtype)
+        np.save(os.path.join(directory, f"{name}.npy"), v)
+    note(f"dumped {len(arrays)} outputs ({total / 2**20:.1f} MiB, {m} of {n} cells) to {directory}")
+
+
 # ------------------------------------------------------------------------------------------------
 class ClockSampler(threading.Thread):
     Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
@@ -372,6 +418,8 @@ def run_b200(a, rank, world, local_rank):
 
     if rank != 0:
         return
+    if a.dump_outputs:
+        dump_outputs(a, out, a.dump_outputs)
     peaks = {}
     try:
         peaks = json.load(open(ROOT / "MEASURED_PEAKS.json"))

@@ -7,7 +7,9 @@ Two sources, both owned by the reference (scverse/scanpy @ fabadb94):
    tests/test_neighbors.py:23-139 (4-point X, distances, umap connectivities, ...).
 2. The in-tree fixture src/scanpy/datasets/10x_pbmc68k_reduced.zarr.zip (zarr v3, sharded,
    zstd): obsm/X_pca, obsp/distances, obsp/connectivities, obs/louvain, uns/neighbors params.
-   Decoded with zipfile + libzstd via ctypes (zarr/anndata are not installed here).
+   Decoded with zipfile + libzstd via ctypes (zarr/anndata are not installed here).  Its
+   `layers/counts` group is also kept as a store (pbmc68k_reduced_counts.zarr.zip) for the
+   zarr reader's test.
 
 Usage:  python tests/golden/make_goldens.py   (writes next to this file)
 """
@@ -93,6 +95,18 @@ def read_zarr_array(z: zipfile.ZipFile, path: str) -> np.ndarray:
     return out
 
 
+def write_counts_store(z: zipfile.ZipFile) -> None:
+    """pbmc68k_reduced_counts.zarr.zip: the fixture's `layers/` entries and `obsm/zarr.json`, byte for byte (the whole
+    fixture is 1.7 MB).  Where the archive holds a key more than once, the last copy is the one readers see and keep."""
+    names = sorted({i.filename for i in z.infolist() if i.filename.startswith("layers/") or i.filename == "obsm/zarr.json"})
+    with zipfile.ZipFile(OUT / "pbmc68k_reduced_counts.zarr.zip", "w") as out:
+        for name in names:
+            info = z.getinfo(name)
+            copy = zipfile.ZipInfo(name, date_time=info.date_time)
+            copy.compress_type = info.compress_type
+            out.writestr(copy, z.read(name))
+
+
 def main() -> None:
     pca_l = literals_from(REF / "tests/test_pca.py", {"A_list", "A_pca", "A_svd"})
     nb_l = literals_from(
@@ -129,6 +143,7 @@ def main() -> None:
     np.savez_compressed(OUT / "pbmc68k_reduced_graph.npz", **fx)
     for k, v in fx.items():
         print(k, v.shape, v.dtype)
+    write_counts_store(z)
 
     # --- preprocessing golden (SURVEY 8f row f2): the reference's tests/test_highly_variable_genes.py:379-421 runs
     # filter_cells -> normalize_total(1e4) -> log1p -> highly_variable_genes(flavor='seurat') on pbmc68k_reduced's

@@ -36,6 +36,8 @@ def test_no_cpu_fallback_without_gpu():
     x = sparse.random(50, 40, density=0.2, format="csr", dtype=np.float32, random_state=0)
     with pytest.raises(_abi.B200Error):
         pp.pca(x, n_comps=5)
+    with pytest.raises(_abi.B200Error):  # zero_center=False is served by the device (TruncatedSVD semantics): no CPU path here
+        pp.pca(_adata(), zero_center=False)
     # the raw C entry point also refuses (no device) instead of computing on the host
     import ctypes
 
@@ -112,8 +114,6 @@ def test_pca_argument_errors_match_reference():
         pp.pca(a, mask_var=np.ones(20, int))
     with pytest.raises(ValueError, match=r"n_components=100 must be between 1 and min\(n_samples, n_features\)=20"):
         pp.pca(a, n_comps=100)  # tests/test_pca.py:292-296
-    with pytest.raises(_abi.B200Error):  # zero_center=False is served by the device (TruncatedSVD semantics): no CPU path here
-        pp.pca(a, zero_center=False)
     with pytest.warns(UserWarning, match="Ignoring svd_solver='randomized'"):
         assert pp._solver_code("randomized", n_vars=100) in (0, 1)  # _pca/__init__.py:451-467
     assert pp._solver_code("covariance_eigh", n_vars=10**6) == 1
@@ -235,14 +235,13 @@ def test_zarr_csr_reader_row_chunks(tmp_path, mode, as_zip):
 
 
 def test_zarr_csr_reader_on_the_reference_fixture():
-    """The reference's own in-tree zarr-v3 fixture (sharded + zstd, written by anndata): `layers/counts` must decode to the
-    same arrays as the independent decoder of tests/golden/make_goldens.py.  Needs /root/reference (build container only)."""
+    """The reference's own in-tree zarr-v3 fixture (sharded + zstd, written by anndata), whose `layers/counts` and `obsm`
+    entries tests/golden keeps byte for byte: `layers/counts` must decode to the same arrays as the independent decoder of
+    tests/golden/make_goldens.py."""
     import sys
     import zipfile
 
-    fixture = Path("/root/reference/src/scanpy/datasets/10x_pbmc68k_reduced.zarr.zip")
-    if not fixture.exists():
-        pytest.skip("reference checkout not present (GPU box)")
+    fixture = Path(__file__).resolve().parent / "golden" / "pbmc68k_reduced_counts.zarr.zip"
     sys.path.insert(0, str(Path(__file__).resolve().parent / "golden"))
     import make_goldens as mg
 
