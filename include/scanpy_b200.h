@@ -286,6 +286,27 @@ int32_t sb2_dense_col_stats(sb2_ctx* ctx, int64_t n, int32_t g, const void* d_x,
 int32_t sb2_dense_scale(sb2_ctx* ctx, int64_t n, int32_t g, void* d_x, int32_t is_f64, const double* d_mean,
                         const double* d_std, const uint8_t* d_mask, int32_t has_max, double max_value);
 
+/* ---- sc.tl.rank_genes_groups (src/scanpy/tools/_rank_genes_groups.py; csrc/rank_genes.cu) ----
+ * Cells carry a group code 0..n_codes-1; code n_codes-1 is the remainder (cells in no selected group).  At most
+ * SB2_RANK_GENES_MAX_GROUPS selected groups (n_codes <= SB2_RANK_GENES_MAX_GROUPS + 1), else SB2_E_UNSUPPORTED.
+ * sb2_rank_genes_group_stats <- the grouped mean / var / count_nonzero of `_basic_stats` (:319-452): for every code q and
+ *   gene j, d_sum = sum of x', d_m2 = sum of (x' - mean)^2 over all n_q cells (implicit zeros included), d_nnz = count of
+ *   x != 0, with x' = expm1(x * expm1_scale) (expm1_scale != 0) or x.  d_rows int32 [n]: the rows ordered by code (stable),
+ *   h_group_offsets int64 [n_codes + 1]: code q owns d_rows[off[q] : off[q + 1]].  Outputs [n_codes x g], bit-reproducible.
+ * sb2_rank_genes_wilcoxon <- the rank sums and tie terms of `wilcoxon` (:505-579), exact integers.  d_codes int32 [n],
+ *   d_group_sizes int64 [n_codes].  ref < 0: ranks over all cells; d_rank2[q][j] = 2 x rank sum of code q, d_tie[q][j] =
+ *   sum over tie runs of gene j of t^3 - t (the same for every q).  ref >= 0: for each q (not ref, not the remainder) ranks
+ *   over the cells of q and ref only; d_rank2[q][j] = 2 x rank sum of q, d_tie[q][j] over those cells; remainder cells take
+ *   no part, rows ref and n_codes-1 are 0.  d_tie uint64 [n_codes x g x 2] = (low, high) 64-bit halves of the 128-bit sum.
+ *   h_stage_ms (may be NULL): float[2] = device ms of the sort and of the rank walk (synchronises the stream). */
+#define SB2_RANK_GENES_MAX_GROUPS 1024
+int32_t sb2_rank_genes_group_stats(sb2_ctx* ctx, int64_t n, int32_t g, const int64_t* d_indptr, const int32_t* d_indices,
+                                   const float* d_data, const int32_t* d_rows, const int64_t* h_group_offsets,
+                                   int32_t n_codes, double expm1_scale, double* d_sum, double* d_m2, int64_t* d_nnz);
+int32_t sb2_rank_genes_wilcoxon(sb2_ctx* ctx, int64_t n, int32_t g, const int64_t* d_indptr, const int32_t* d_indices,
+                                const float* d_data, int64_t nnz, const int32_t* d_codes, const int64_t* d_group_sizes,
+                                int32_t n_codes, int32_t ref, int64_t* d_rank2, uint64_t* d_tie, float* h_stage_ms);
+
 #ifdef __cplusplus
 }
 #endif

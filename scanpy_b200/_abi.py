@@ -119,7 +119,13 @@ SIGNATURES = {
     "sb2_log1p_f32": (c_int32, [c_void_p, c_int64, c_void_p, c_double]),
     "sb2_csr_col_sums_f32": (c_int32, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int32, c_double, c_void_p,
                                        c_void_p]),
+    "sb2_rank_genes_group_stats": (c_int32, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                             c_int32, c_double, c_void_p, c_void_p, c_void_p]),
+    "sb2_rank_genes_wilcoxon": (c_int32, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
+                                          c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
 }
+
+RANK_GENES_MAX_GROUPS = 1024  # SB2_RANK_GENES_MAX_GROUPS in include/scanpy_b200.h
 
 _lib = None
 

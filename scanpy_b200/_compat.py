@@ -1,8 +1,8 @@
 """Small host-side pieces of scanpy's runtime that the three hot-path functions lean on.
 
 * `MiniAnnData` — a duck-typed stand-in for `anndata.AnnData` (anndata is not installed in the build
-  image).  The public functions only use `.X .obs .var .obsm .varm .obsp .uns .n_obs .n_vars
-  .shape .is_view .copy()` and `adata[:, mask]`, so a real AnnData works unchanged.
+  image).  The public functions only use `.X .obs .var .var_names .obsm .varm .obsp .uns .layers .raw
+  .n_obs .n_vars .shape .is_view .copy()` and `adata[:, mask]`, so a real AnnData works unchanged.
 * `settings` — the two constants the path reads (`N_PCS`, `n_jobs`; src/scanpy/_settings/__init__.py:83,132)
   plus verbosity-free logging with the reference's message texts (src/scanpy/logging.py:100-131).
 * `accepts_legacy_random_state` — the `random_state=` <-> `rng=` shim of
@@ -96,8 +96,13 @@ class MiniAnnData:
         self.obsp = _AxisArrays(obsp or {})
         self.uns = dict(uns or {})
         self.layers = {}
+        self.raw = None  # anything with .X and .var_names (e.g. another MiniAnnData), as `anndata.AnnData.raw`
         self.is_view = False
         self.isbacked = False
+
+    @property
+    def var_names(self) -> pd.Index:
+        return self.var.index
 
     @property
     def shape(self):
@@ -114,9 +119,11 @@ class MiniAnnData:
     def copy(self):
         import copy
 
-        return MiniAnnData(self.X.copy(), self.obs.copy(), self.var.copy(),
-                           {k: v.copy() for k, v in self.obsm.items()}, {k: v.copy() for k, v in self.varm.items()},
-                           {k: v.copy() for k, v in self.obsp.items()}, copy.deepcopy(self.uns))
+        new = MiniAnnData(self.X.copy(), self.obs.copy(), self.var.copy(),
+                          {k: v.copy() for k, v in self.obsm.items()}, {k: v.copy() for k, v in self.varm.items()},
+                          {k: v.copy() for k, v in self.obsp.items()}, copy.deepcopy(self.uns))
+        new.raw = self.raw.copy() if self.raw is not None else None
+        return new
 
     def __getitem__(self, idx):
         if not (isinstance(idx, tuple) and len(idx) == 2 and isinstance(idx[0], slice) and idx[0] == slice(None)):

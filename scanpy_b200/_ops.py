@@ -497,3 +497,77 @@ def umap_layout(adj, *, n_components: int, n_epochs: int, a: float, b: float, ga
                                       float(a), float(b), float(gamma), float(initial_alpha), int(negative_sample_rate),
                                       int(seed), ptr(emb)))
     return _to_host(emb)
+
+
+# ------------------------------------------------------------------------------------------ rank_genes_groups
+def _csr_f32(x):
+    """scipy CSR -> the same matrix with float32 data and canonical (summed duplicate) entries."""
+    x = x.tocsr()
+    if x.dtype != np.float32:
+        x = x.astype(np.float32)
+    if not x.has_canonical_format:
+        x = x.copy()
+        x.sum_duplicates()
+    return x
+
+
+def rank_genes_group_stats(x, codes: np.ndarray, n_codes: int, *, expm1_scale: float = 0.0, ctx=None):
+    """Per (code, gene) sums, M2 = sum (x' - mean)^2 and counts of x != 0 over a scipy CSR, x' = expm1(x * expm1_scale)
+    (expm1_scale != 0) or x; codes int [n] in 0..n_codes-1.  -> (sum float64, m2 float64, nnz int64), each [n_codes, g]."""
+    torch = _torch()
+    ctx = ctx or _abi.default_context()
+    x = _csr_f32(x)
+    n, g = x.shape
+    codes = np.asarray(codes, dtype=np.int32)
+    rows = np.argsort(codes, kind="stable").astype(np.int32)
+    offsets = np.zeros(n_codes + 1, np.int64)
+    np.cumsum(np.bincount(codes, minlength=n_codes), out=offsets[1:])
+    d_indptr, d_indices, d_data = csr_to_device(x)
+    d_rows = _to_device(rows)
+    s = torch.empty((n_codes, g), dtype=torch.float64, device="cuda")
+    m2 = torch.empty((n_codes, g), dtype=torch.float64, device="cuda")
+    nnz = torch.empty((n_codes, g), dtype=torch.int64, device="cuda")
+    check(ctx.lib.sb2_rank_genes_group_stats(ctx.handle, n, g, ptr(d_indptr), ptr(d_indices), ptr(d_data), ptr(d_rows),
+                                             ptr(offsets), int(n_codes), float(expm1_scale), ptr(s), ptr(m2), ptr(nnz)))
+    return _to_host(s, m2, nnz)
+
+
+def tie_terms_to_int(tie: np.ndarray) -> np.ndarray:
+    """(low, high) uint64 halves [..., 2] -> exact Python-int object array [...]."""
+    lo, hi = tie[..., 0], tie[..., 1]
+    out = np.empty(lo.shape, dtype=object)
+    for idx in np.ndindex(lo.shape):
+        out[idx] = (int(hi[idx]) << 64) | int(lo[idx])
+    return out
+
+
+def tie_terms_to_f64(tie: np.ndarray) -> np.ndarray:
+    """(low, high) uint64 halves [..., 2] -> float64 [...] (the nearest double to within two roundings)."""
+    return tie[..., 1].astype(np.float64) * 2.0**64 + tie[..., 0].astype(np.float64)
+
+
+def rank_genes_wilcoxon(x, codes: np.ndarray, n_codes: int, *, ref: int = -1, stage_ms: list | None = None, ctx=None):
+    """Wilcoxon rank sums and tie terms on the device (sb2_rank_genes_wilcoxon); codes int [n] in 0..n_codes-1, code
+    n_codes-1 the remainder.  ref < 0: ranks over all cells; else, per code, over that code and `ref` only.
+    -> (rank2 int64 [n_codes, g]: twice the rank sums, tie uint64 [n_codes, g, 2]: sum of t^3 - t as low/high halves).
+    `stage_ms`, if a list, receives the device milliseconds of the sort and of the rank walk."""
+    from ctypes import c_float
+
+    torch = _torch()
+    ctx = ctx or _abi.default_context()
+    x = _csr_f32(x)
+    n, g = x.shape
+    codes = np.asarray(codes, dtype=np.int32)
+    sizes = np.bincount(codes, minlength=n_codes).astype(np.int64)
+    d_indptr, d_indices, d_data = csr_to_device(x)
+    d_codes, d_sizes = _to_device(codes), _to_device(sizes)
+    rank2 = torch.empty((n_codes, g), dtype=torch.int64, device="cuda")
+    tie = torch.empty((n_codes, g, 2), dtype=torch.int64, device="cuda")
+    ms = (c_float * 2)() if stage_ms is not None else None
+    check(ctx.lib.sb2_rank_genes_wilcoxon(ctx.handle, n, g, ptr(d_indptr), ptr(d_indices), ptr(d_data), int(x.nnz),
+                                          ptr(d_codes), ptr(d_sizes), int(n_codes), int(ref), ptr(rank2), ptr(tie),
+                                          ms))
+    if stage_ms is not None:
+        stage_ms[:] = [float(ms[0]), float(ms[1])]
+    h_rank2, h_tie = _to_host(rank2, tie)
+    return h_rank2, h_tie.view(np.uint64)

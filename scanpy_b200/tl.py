@@ -181,3 +181,4 @@ def _natkey(s: str):
 
 
 from ._graph_tools import diffmap, paga, umap  # noqa: E402,F401  (SURVEY.md 8f rows f1, f3)
+from ._rank_genes import rank_genes_groups  # noqa: E402,F401
